@@ -9,20 +9,25 @@ scaling), bf16 compute with fp32 master weights, synthetic tokens, random-init w
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 \
         --master-port 29500 bench.py --gpus 8 --steps 20 --warmup 5
     python bench.py --impl reference ...      # the unmodified reference (needs OneFlow)
+    python bench.py --steps 20 --warmup 5 --dump-outputs output/bench   # + what the last timed step computed (.npy)
 
 Prints ONE JSON line (rank 0).  ``value`` is device-timed (CUDA events, max over ranks) over exactly
 ``--steps`` full training steps (fwd + bwd + grad sync + optimizer); ``e2e`` repeats the
 measurement through the public trainer API including the per-step pinned-host→device input copy and
-the device→host loss read.
+the device→host loss read.  Inputs and initial weights are seeded, so two builds run with the same
+arguments can be compared output for output through ``--dump-outputs``.  Nothing is written into the
+source tree: the trainer's output directory is a temporary one.
 """
 from __future__ import annotations
 
 import argparse
 import json
 import os
+import shutil
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -87,7 +92,12 @@ def parse_args():
     ap.add_argument("--fp8", type=int, default=0,
                     help="1: forward GEMMs with E4M3 operands (experiment; the headline number is the bf16 default — "
                          "the JSON line then says dtype fp8-fwd/bf16-bwd)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps write what the last one computed (its loss dict and a seeded sample of "
+                         "the updated model state, rank 0) as DIR/<name>.npy, float32")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     spec = MODELS[a.model]
     for k in ("layers", "hidden", "heads", "seq"):
         if not getattr(a, k):
@@ -260,7 +270,7 @@ def build_cfg(args, lay):
     cfg.train.amp.enabled = True
     cfg.train.evaluation.enabled = False
     cfg.train.checkpointer.period = 10 ** 9
-    cfg.train.output_dir = os.path.join(REPO, "output", "bench")
+    cfg.train.output_dir = args.output_dir
     cfg.train.cuda_graphs.enabled = bool(args.graphs)
     cfg.train.dist.tensor_parallel_size = lay["tp"]
     cfg.train.dist.pipeline_parallel_size = lay["pp"]
@@ -276,9 +286,37 @@ def build_cfg(args, lay):
     return cfg
 
 
-def measure_native(args, lay, world, rank, local_rank, steps, warmup, with_e2e, clock_sampler=None):
+DUMP_SAMPLES_PER_TENSOR = 4096     # ~3 MB of float32 for the headline model (its whole state would be ~1.4 GB)
+
+
+def dump_outputs(out_dir, loss, model):
+    """Write what a training step computed as ``out_dir/<name>.npy`` (float32): every entry of the loss dict the step
+    returns (``lm_loss.npy``) and ``state_sample.npy``, the same seeded sample of ``DUMP_SAMPLES_PER_TENSOR`` elements
+    of every floating-point tensor of the updated state dict (all of a smaller tensor), concatenated in state-dict
+    order."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in (loss or {}).items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v.detach().float().cpu().numpy())
+    g = torch.Generator().manual_seed(0)
+    parts = []
+    for t in model.state_dict().values():
+        if not t.is_floating_point():
+            continue
+        flat = t.detach().reshape(-1)
+        n = flat.numel()
+        k = DUMP_SAMPLES_PER_TENSOR
+        idx = torch.arange(n) if n <= k else torch.randint(0, n, (k,), generator=g)
+        parts.append(flat[idx.to(flat.device)].float().cpu())
+    np.save(os.path.join(out_dir, "state_sample.npy"), torch.cat(parts).numpy())
+
+
+def measure_native(args, lay, world, rank, local_rank, steps, warmup, with_e2e, clock_sampler=None, dump_dir=""):
     """Build the trainer for ``lay`` through the public API, time ``steps`` optimizer steps on the device (CUDA events,
-    max over ranks) and optionally the end-to-end loop through ``trainer.run_step()``."""
+    max over ranks) and optionally the end-to-end loop through ``trainer.run_step()``.  With ``dump_dir``, rank 0 then
+    writes what the last timed step computed there (:func:`dump_outputs`)."""
     import gc
     import logging
 
@@ -388,6 +426,8 @@ def measure_native(args, lay, world, rank, local_rank, steps, warmup, with_e2e, 
     if world > 1:
         dist.all_reduce(lv, op=dist.ReduceOp.MAX)
     res["final_loss"] = float(lv) if float(lv) > -1e29 else None
+    if dump_dir and rank == 0:        # before the end-to-end loop trains on
+        dump_outputs(dump_dir, loss, step.model.module if hasattr(step.model, "module") else step.model)
 
     # ---- end to end through the trainer API: loader (pinned host) → H2D → step → loss D2H, every step ---------------
     if with_e2e:
@@ -578,10 +618,13 @@ def main():
     if local_rank == 0 and os.path.exists(_extras_flag_path()):
         os.remove(_extras_flag_path())       # before the rendezvous: no rank can have raised it yet in this launch
     _dutil.init_process_group("cuda")        # torchrun environment → NCCL (+ gloo for host objects)
+    # the trainer's output directory (config dump, log): the source tree may be read-only
+    args.output_dir = tempfile.mkdtemp(prefix="libai_b200_bench_")
 
     primary = layout_of(args, world)
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    main_res = measure_native(args, primary, world, rank, local_rank, args.steps, args.warmup, not args.no_e2e, sampler)
+    main_res = measure_native(args, primary, world, rank, local_rank, args.steps, args.warmup, not args.no_e2e, sampler,
+                              args.dump_outputs)
 
     layouts = {main_res["parallelism"]: {k: main_res[k] for k in ("value", "ms_per_step", "cuda_graphs", "gpu_launches",
                                                                   "host_enqueue_ms_per_step", "global_batch")}}
@@ -670,6 +713,7 @@ def main():
     watch.stop()
 
     emit()
+    shutil.rmtree(args.output_dir, ignore_errors=True)
     if world > 1:
         dist.destroy_process_group()
     return 0

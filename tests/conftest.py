@@ -9,7 +9,7 @@ if REPO not in sys.path:
 
 
 def pytest_configure(config):
-    config.addinivalue_line("markers", "gpu: test needs a CUDA device (run on a B200 via gpurun)")
+    config.addinivalue_line("markers", "gpu: test needs a CUDA device (a B200)")
 
 
 def pytest_collection_modifyitems(config, items):
@@ -21,6 +21,22 @@ def pytest_collection_modifyitems(config, items):
     for item in items:
         if "gpu" in item.keywords:
             item.add_marker(skip)
+
+
+@pytest.hookimpl(hookwrapper=True)
+def pytest_runtest_protocol(item, nextitem):
+    """Tests not marked ``gpu`` are the CPU tier: they run on the CPU also where a GPU is visible (layers would otherwise
+    default to it), in this process and in the processes they start, so that they check the same code on every
+    machine.  Set around the whole protocol so that module-scoped fixtures are built on the CPU too."""
+    if "gpu" in item.keywords:
+        yield
+        return
+    import torch
+
+    with pytest.MonkeyPatch.context() as mp:
+        mp.setenv("CUDA_VISIBLE_DEVICES", "")
+        mp.setattr(torch.cuda, "is_available", lambda: False)
+        yield
 
 
 @pytest.fixture(autouse=True)

@@ -16,6 +16,34 @@ def test_reference_arm_reports_unavailable():
     assert "unavailable" in line or "value" in line      # (a value only if OneFlow were importable)
 
 
+def test_bench_rejects_zero_steps():
+    r = subprocess.run([sys.executable, "bench.py", "--steps", "0"], cwd=REPO, capture_output=True, text=True, timeout=300)
+    assert r.returncode == 2 and "--steps" in r.stderr
+
+
+def test_dump_outputs_writes_a_seeded_float32_sample(tmp_path):
+    """`bench.py --dump-outputs`: the loss dict and the same sample of the model state on every call."""
+    import numpy as np
+    import torch
+
+    sys.path.insert(0, REPO)
+    import bench
+
+    torch.manual_seed(0)
+    model = torch.nn.Sequential(torch.nn.Linear(100, 100), torch.nn.LayerNorm(100)).bfloat16()
+    model.register_buffer("steps", torch.tensor(3))          # integer state is not sampled
+    loss = {"lm_loss": torch.tensor(2.5)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), loss, model)
+    assert sorted(os.listdir(tmp_path / "a")) == ["lm_loss.npy", "state_sample.npy"]
+    a, b = np.load(tmp_path / "a" / "state_sample.npy"), np.load(tmp_path / "b" / "state_sample.npy")
+    assert a.dtype == np.float32 and a.shape == (bench.DUMP_SAMPLES_PER_TENSOR + 3 * 100,) and np.array_equal(a, b)
+    w = model[0].weight.detach().float().flatten().numpy()
+    assert np.isin(a[:bench.DUMP_SAMPLES_PER_TENSOR], w).all()              # sampled from the large tensor
+    assert np.array_equal(a[bench.DUMP_SAMPLES_PER_TENSOR:][:100], model[0].bias.detach().float().numpy())   # small: whole
+    assert np.load(tmp_path / "a" / "lm_loss.npy") == np.float32(2.5)
+
+
 _WATCHDOG_SCRIPT = r"""
 import json, os, sys, time
 sys.path.insert(0, {repo!r})

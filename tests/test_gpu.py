@@ -190,14 +190,23 @@ def test_smoke_entry_point():
     __graft_entry__.smoke()
 
 
-def test_bench_contract():
-    r = _run([sys.executable, "bench.py", "--steps", "2", "--warmup", "3"], timeout=1200)
+def test_bench_contract(tmp_path):
+    import numpy as np
+
+    dump = tmp_path / "outputs"
+    r = _run([sys.executable, "bench.py", "--steps", "2", "--warmup", "3", "--dump-outputs", str(dump)], timeout=1200)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
     line = json.loads(r.stdout.strip().splitlines()[-1])
     for key in ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
                 "vs_baseline", "dtype", "data", "config", "clocks", "e2e", "gpu_launches"):
         assert key in line, key
     assert line["value"] > 0 and line["gpu_launches"] > 0 and line["e2e"]["h2d_bytes_per_step"] > 0
+    # what the last timed step computed: its loss (the line's final_loss) and a sample of the updated weights
+    assert sorted(os.listdir(dump)) == ["lm_loss.npy", "state_sample.npy"]
+    assert sum(os.path.getsize(dump / f) for f in os.listdir(dump)) <= 64 << 20
+    loss, state = np.load(dump / "lm_loss.npy"), np.load(dump / "state_sample.npy")
+    assert loss.dtype == state.dtype == np.float32 and np.isfinite(state).all()
+    assert abs(float(loss) - line["final_loss"]) < 1e-6 * abs(line["final_loss"])
     ref = _run([sys.executable, "bench.py", "--impl", "reference"])
     assert ref.returncode == 0 and json.loads(ref.stdout.strip().splitlines()[-1])["impl"] == "reference"
 
